@@ -21,6 +21,14 @@ N = 8 is exactly BASELINE configs[3] (1024^3 ComplexF64, process grid (4,2)).
 
   python bench.py [--gpus N] [--steps K] [--warmup W]        # this framework
   python bench.py --impl reference ...                       # CPU port of the reference path
+  python bench.py ... --dump-outputs bench_outputs   # also write what the last timed step computed
+
+--dump-outputs DIR writes DIR/ux.npy, uy.npy, uz.npy (suffix _rank<r> when N > 1): the x-, y-
+and z-pencil arrays as the last timed step left them, i.e. what the four transpose! calls hand
+their caller, each a fixed sample when the whole would exceed 48 MiB in all.  The inputs are
+seeded, so two builds run with the same arguments can be compared file by file.  Only uy and
+uz carry computed data: the step is a round trip, so ux is the seeded input again (which the
+round_trip_bit_exact check already confirms); a match in ux says nothing about the kernels.
 """
 import argparse
 import ctypes as C
@@ -142,6 +150,25 @@ class ClockSampler:
         return {"sm_mhz": sm[len(sm) // 2] if sm else None, "sm_max_mhz": max(mx) if mx else None,
                 "samples": len(sm), "window": window, "region_ms": round((t1 - t0) * 1e3, 1),
                 "reasons": sorted(reasons)}
+
+
+DUMP_BYTES = 48 << 20  # all --dump-outputs files of one run together
+
+
+def dump_outputs(outdir, arrays, rank, n, torch):
+    """Saves each (name, PencilArray) as OUTDIR/<name>.npy: the parent (memory-order) array,
+    flattened; complex as (count, 2) real.  An array above its share of DUMP_BYTES is reduced
+    to a sample at sorted positions drawn from a fixed seed, the same in every run."""
+    import numpy as np
+    os.makedirs(outdir, exist_ok=True)
+    for name, u in arrays:
+        flat = u.data.reshape(-1)
+        keep = DUMP_BYTES // (len(arrays) * n * flat.element_size())
+        if flat.numel() > keep:
+            idx = np.sort(np.random.default_rng(0).choice(flat.numel(), keep, replace=False))
+            flat = flat[torch.from_numpy(idx).to(flat.device)]
+        out = (torch.view_as_real(flat) if flat.is_complex() else flat).cpu().numpy()
+        np.save(os.path.join(outdir, name + (f"_rank{rank}" if n > 1 else "") + ".npy"), out)
 
 
 def workload_name(n, wl="cfg4"):
@@ -647,6 +674,8 @@ def run_b200(args):
             leg_ms[i] += legs[k][i].elapsed_time(legs[k][i + 1]) / args.steps
     leg_ms = [max_over_ranks(x) for x in leg_ms]
     ok = bool(torch.equal(ux.data.view(torch.uint8), orig.view(torch.uint8)))
+    if args.dump_outputs:  # before the placement check below overwrites the arrays
+        dump_outputs(args.dump_outputs, [("ux", ux), ("uy", uy), ("uz", uz)], rank, n, torch)
     gbytes = math.prod(dims) * isz
     value = 4 * gbytes / GIB / (ms * 1e-3)
 
@@ -971,9 +1000,15 @@ def main():
     ap.add_argument("--host-chunk-mib", type=int, default=None, help="e2e: tunable host_chunk_bytes")
     ap.add_argument("--quick", action="store_true", help="skip the side measurements (kernels, configs[1])")
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the arrays the last timed step computed as DIR/<name>.npy")
     args = ap.parse_args()
     if args.gpus not in (1, 2, 4, 8):
         raise SystemExit("--gpus must be 1, 2, 4 or 8")
+    if args.steps < 1:
+        raise SystemExit("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        raise SystemExit("--dump-outputs writes the B200 arm's arrays: not with --impl reference")
     if args.warmup < 3:
         args.warmup = 3
     if args.impl == "reference":

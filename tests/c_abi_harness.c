@@ -6,6 +6,7 @@
  *     parent(u)[perm * I] == global[I]        (arrays.jl:19-31, 327-337)
  * evaluated with naive loops here.  Exit codes: 0 ok, 2 no GPU (the library
  * refused: there is no CPU fallback), 1 anything else.
+ * Usage: c_abi_harness FILE -- FILE is the scratch path of the PencilIO check.
  * Built and run by tests/test_c_abi_harness.py.
  */
 #include <stdint.h>
@@ -40,7 +41,11 @@ static int64_t off(const int* perm, const int64_t* n, const int64_t* I) {
   return o;
 }
 
-int main(void) {
+int main(int argc, char** argv) {
+  if (argc != 2) {
+    fprintf(stderr, "usage: %s SCRATCH_FILE\n", argv[0]);
+    return 1;
+  }
   const int64_t n[3] = {24, 20, 12};
   const int64_t pdims[2] = {1, 1};
   const int dx[2] = {2, 3}, dy[2] = {1, 3}, dz[2] = {1, 2};
@@ -144,7 +149,7 @@ int main(void) {
   /* PencilIO layout: the file is the global array in the pencil's MEMORY order
    * (mpi_io.jl:372-380): written from the device, checked byte for byte, read back */
   {
-    const char* path = "/tmp/pa_c_harness.bin";
+    const char* path = argv[1];
     FILE* f = fopen(path, "wb");
     if (!f) return 1;
     fclose(f);

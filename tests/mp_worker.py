@@ -16,6 +16,7 @@ part bit for bit.
 """
 import os
 import sys
+import tempfile
 
 import numpy as np
 import torch
@@ -100,6 +101,12 @@ def main():
         dist.init_process_group("gloo")
         comm = pa.Comm(dist.get_rank(), dist.get_world_size())
     rank, world = comm.rank, comm.size
+    # the directory every rank writes its PencilIO file to: the test's own, or (when the
+    # worker is started by hand) one that rank 0 makes and tells the others about
+    scratch = [os.environ.get("PA_TEST_SCRATCH") or (tempfile.mkdtemp(prefix="pa_mp_worker_")
+                                                     if rank == 0 else None)]
+    dist.broadcast_object_list(scratch, src=0)
+    scratch = scratch[0]
     ran = 0
     extra_cases = []
     if mode != "gloo":
@@ -269,7 +276,7 @@ def main():
             u = pa.PencilArray.undef(tdt, pen, *extra)
             u.data.view(torch.uint8).reshape(-1).copy_(torch.from_numpy(
                 np.ascontiguousarray(mine.data.reshape(-1, order="F")).view(np.uint8).copy()))
-            fname = f"/tmp/pa_io_{os.environ.get('MASTER_PORT', '0')}_{case['name']}.bin"
+            fname = os.path.join(scratch, f"pa_io_{case['name']}.bin")
             with pa.open_(pa.MPIIODriver(), fname, comm, write=True, create=True) as ff:
                 ff.write("u", u, chunks=False)
                 ff.write("u_chunks", u, chunks=True)
@@ -292,6 +299,8 @@ def main():
                 os.remove(fname)
                 os.remove(fname + ".json")
     dist.barrier()
+    if rank == 0 and not os.environ.get("PA_TEST_SCRATCH"):
+        os.rmdir(scratch)
     if rank == 0:
         print(f"MP_WORKER_OK mode={mode} world={world} cases={ran} launches={pa.launch_count()}")
     dist.destroy_process_group()

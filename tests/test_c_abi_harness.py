@@ -26,13 +26,15 @@ def _build(tmp_path):
 def test_c_harness_refuses_without_gpu(tmp_path):
     if torch.cuda.is_available():
         pytest.skip("GPU present")
-    out = subprocess.run([_build(tmp_path)], capture_output=True, text=True, timeout=120)
+    out = subprocess.run([_build(tmp_path), str(tmp_path / "io.bin")], capture_output=True, text=True,
+                         timeout=120)
     assert out.returncode == 2, (out.stdout, out.stderr)
     assert "no CUDA device" in out.stdout
 
 
 @pytest.mark.gpu
 def test_c_harness_on_gpu(tmp_path):
-    out = subprocess.run([_build(tmp_path)], capture_output=True, text=True, timeout=300)
+    out = subprocess.run([_build(tmp_path), str(tmp_path / "io.bin")], capture_output=True, text=True,
+                         timeout=300)
     assert out.returncode == 0, (out.stdout, out.stderr)
     assert "C ABI harness OK" in out.stdout

@@ -20,7 +20,7 @@ import pencilarrays_b200 as pa
 from pencilarrays_b200._lib import lib, check
 from pencilarrays_b200.transpositions import _Plan
 from oracle import pencil_oracle as O
-from util import CASES, DTYPES, beq, build_chain
+from util import CASES, DTYPES, beq, build_chain, golden_nbytes, matches_golden
 from gpu_util import TORCH_OF, dev_bytes, host_bytes, emulate_transpose_gpu, ptr
 
 pytestmark = pytest.mark.gpu
@@ -346,10 +346,10 @@ def test_gpu_path_against_committed_golden_fixtures():
         for k in range(1, len(steps)):
             plans = [_Plan(steps[k - 1][r][0], steps[k][r][0], extra, it, pa.PointToPoint())
                      for r in range(len(ranks))]
-            wants = [z[f"step{k}_rank{r}"] for r in range(len(ranks))]
-            nxt = [torch.full((max(1, w.size),), 0xA5, dtype=torch.uint8, device="cuda") for w in wants]
+            sizes = [golden_nbytes(z, k, r) for r in range(len(ranks))]
+            nxt = [torch.full((max(1, n),), 0xA5, dtype=torch.uint8, device="cuda") for n in sizes]
             emulate_transpose_gpu(plans, cur, nxt, fused_self=True)
             torch.cuda.synchronize()
-            for r, w in enumerate(wants):
-                assert host_bytes(nxt[r])[:w.size].tobytes() == w.tobytes(), (f, k, r)
-            cur = [t[:max(1, w.size)] for t, w in zip(nxt, wants)]
+            for r, n in enumerate(sizes):
+                assert matches_golden(z, k, r, host_bytes(nxt[r])[:n]), (f, k, r)
+            cur = [t[:max(1, n)] for t, n in zip(nxt, sizes)]

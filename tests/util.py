@@ -8,6 +8,7 @@ format, not a fallback of the product.
 from __future__ import annotations
 
 import ctypes as C
+import hashlib
 import math
 import os
 import sys
@@ -29,6 +30,24 @@ def beq(a, b) -> bool:
     a = np.ascontiguousarray(a)
     b = np.ascontiguousarray(b)
     return a.shape == b.shape and a.dtype.itemsize == b.dtype.itemsize and a.tobytes() == b.tobytes()
+
+
+def golden_nbytes(z, k, r) -> int:
+    """Length in bytes of the output of step k on rank r in a tests/golden fixture."""
+    key = f"step{k}_rank{r}"
+    return int(z[key + "_nbytes"]) if key + "_pos" in z.files else z[key].size
+
+
+def matches_golden(z, k, r, got) -> bool:
+    """`got` (the whole uint8 output of step k on rank r) against a tests/golden fixture:
+    byte for byte where the fixture holds all of it; otherwise at the stored sample
+    positions and through the SHA-256 of all bytes (see tests/golden/make_golden.py)."""
+    key = f"step{k}_rank{r}"
+    got = np.ascontiguousarray(got).view(np.uint8).reshape(-1)
+    if key + "_pos" not in z.files:
+        return got.tobytes() == z[key].tobytes()
+    return (got.size == int(z[key + "_nbytes"]) and got[z[key + "_pos"]].tobytes() == z[key].tobytes()
+            and hashlib.sha256(got.tobytes()).digest() == z[key + "_sha256"].tobytes())
 
 
 def apply_block(desc, src_flat: np.ndarray, dst_flat: np.ndarray):
